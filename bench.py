@@ -2,7 +2,7 @@
 """
 bench.py -- map_cells_to_space iterations/sec on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c4|c5] [--precision bf16|fp32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c4|c5] [--precision bf16|fp32] [--dump-outputs DIR]
     python bench.py --impl reference ...      # the reference's own CPU path (unmodified Mapper from oracle/_ref), full size
 
 A "step" is one optimizer iteration (loss, backward, Adam) of the hot path on synthetic
@@ -144,6 +144,37 @@ def mem_available_gb():
     except OSError:
         pass
     return 0.0
+
+
+def reference_present():
+    """The reference legs need the unmodified reference Mapper that build() copies into oracle/_ref where the reference
+    tree exists; without it they are reported as not measured."""
+    from oracle import build_ref
+    return os.path.exists(build_ref.REF_DST) or os.path.exists(build_ref.REF_SRC)
+
+
+def dump_outputs(out_dir, eng, n_rows, n_voxels, hist, budget=64_000_000):
+    """What the timed path computed, as .npy files for comparing two builds output for output: one float32 file per loss
+    term a Mapper.train caller receives (total_loss.npy, main_loss.npy, ...), one value per timed step, and softmax(M) after
+    the last timed step (mapping.npy, float32).  A term whose lambda is 0 is NaN by the reference's convention (x / lambda)
+    and is not written.  When the whole mapping does not fit the budget it is a fixed seeded sample of rows, sorted,
+    listed in mapping_rows.npy (float64)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    c = eng.cfg
+    terms = {"total_loss": 1.0, "main_loss": c.lambda_g1, "vg_reg": c.lambda_g2, "kl_reg": c.lambda_d, "entropy_reg": c.lambda_r}
+    losses = {name: np.ascontiguousarray(hist[:, col]) for col, (name, lam) in enumerate(terms.items()) if lam != 0}
+    k = int(min(n_rows, (budget - sum(x.nbytes for x in losses.values())) // (4 * n_voxels + 8)))
+    rows = np.arange(n_rows) if k == n_rows else np.sort(np.random.default_rng(0).choice(n_rows, k, replace=False))
+    P = torch.empty((n_rows, n_voxels), dtype=torch.float32, device="cuda")
+    eng.get_mapping(P)
+    torch.cuda.synchronize()
+    np.save(os.path.join(out_dir, "mapping.npy"), P[torch.from_numpy(rows).cuda()].cpu().numpy())
+    del P
+    torch.cuda.empty_cache()
+    np.save(os.path.join(out_dir, "mapping_rows.npy"), rows.astype(np.float64))
+    for name, x in losses.items():
+        np.save(os.path.join(out_dir, name + ".npy"), x)
 
 
 def reference_kwargs(name, inp, device, random_state=42):
@@ -347,6 +378,8 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-refgpu", action="store_true", help="skip the PyTorch-GPU comparator and the parity legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed steps computed to DIR/*.npy (rank 0: its own cells; at most 64 MB)")
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3)
 
@@ -468,6 +501,8 @@ def main():
         parity["max_abs_diff_vs_expected"] = float(np.max(np.abs(hist[:, 0].astype(np.float64) - np.array(exp["total_loss"][:n_total]))))
     if os.environ.get("TGB200_RECORD_EXPECTED") and rank == 0 and world == 1:
         parity["recorded_trajectory"] = [float(x) for x in hist[:, 0]]
+    if a.dump_outputs and rank == 0:      # before the profiled steps below move the mapping on
+        dump_outputs(a.dump_outputs, eng, r1 - r0, V, hist[a.warmup:])
 
     # ---------------- roofline of the dominant kernel, timed live with CUDA events on this stream
     prof = {}
@@ -586,12 +621,13 @@ def main():
 
     # ---------------- reference legs (rank 0, single GPU): PyTorch-GPU comparator + parity at the benchmark size, CPU sample
     refgpu = x3 = None
-    if rank == 0 and world == 1 and not a.no_refgpu:
+    have_ref = reference_present()
+    if rank == 0 and world == 1 and not a.no_refgpu and have_ref:
         torch.cuda.empty_cache()
         refgpu, par_ref, x3 = reference_gpu_legs(a, inp, local, make_engine, n_total)
         parity["vs_reference_gpu"] = par_ref
     cpu = None
-    if rank == 0 and world == 1 and not a.no_cpu:
+    if rank == 0 and world == 1 and not a.no_cpu and have_ref:
         cpu = reference_cpu_sample(a.workload)
 
     if rank == 0:
@@ -608,6 +644,7 @@ def main():
                                              "lives in ncclMemAlloc memory registered with the communicator (NVLS in-switch reduction on user buffers)"}
                                if world > 1 else None),
                 "parity": parity, "reference_gpu": refgpu,
+                "reference_note": None if have_ref else "oracle/_ref/mapping_optimizer.py absent: reference legs not measured",
                 "vs_reference_gpu": (value / refgpu["value"]) if refgpu else None, "bf16x3": x3}
         print(json.dumps(line))
     if world > 1:

@@ -1,15 +1,11 @@
 """Shared helpers for the parity tests (oracle is the checker, never the product)."""
+import hashlib
 import os
 
 import numpy as np
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 GOLDEN_CASES = ["cells_default", "cells_nodensity", "cells_regs", "clusters", "cells_spatial"]
-# The reference's one-file hot path: the tree itself where it exists (this container), else the verbatim copy that
-# oracle/build_ref.py left in oracle/_ref/ (git-ignored; it travels to the GPU box with the snapshot).
-_REF_CANDIDATES = ["/root/reference/tangram/mapping_optimizer.py",
-                   os.path.join(os.path.dirname(GOLDEN_DIR.rstrip(os.sep)), "..", "oracle", "_ref", "mapping_optimizer.py")]
-REFERENCE_FILE = next((os.path.abspath(p) for p in _REF_CANDIDATES if os.path.exists(p)), _REF_CANDIDATES[0])
 
 
 def load_golden(name):
@@ -39,12 +35,9 @@ def max_rel(a, b):
     return float(np.max(np.abs(a - b) / np.maximum(np.abs(b), 1e-12)))
 
 
-def load_reference_module():
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("ref_mapping_optimizer", REFERENCE_FILE)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+def sha256_f32(a):
+    """Digest of an array's float32 bytes (how the golden files pin the reference's initial mapping)."""
+    return hashlib.sha256(np.ascontiguousarray(a, dtype=np.float32).tobytes()).hexdigest()
 
 
 def assert_same_print(ours, ref):

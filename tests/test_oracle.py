@@ -1,6 +1,5 @@
 """Pin the oracle (oracle/tangram_oracle.py) against vectors produced by the real
-reference (tests/golden/make_golden.py), and -- where /root/reference exists -- against
-the live reference.  CPU only."""
+reference (tests/golden/make_golden.py, tests/golden/make_live_reference_golden.py).  CPU only."""
 import contextlib
 import io
 import os
@@ -10,7 +9,7 @@ import pytest
 import torch
 
 from oracle.tangram_oracle import OracleMapper, synthetic_inputs
-from tests.helpers import assert_same_print, GOLDEN_CASES, REFERENCE_FILE, load_golden, load_reference_module, max_rel, rel_fro
+from tests.helpers import assert_same_print, GOLDEN_CASES, GOLDEN_DIR, load_golden, max_rel, rel_fro, sha256_f32
 
 
 @pytest.mark.parametrize("name", GOLDEN_CASES)
@@ -70,22 +69,17 @@ def test_oracle_float64_gradient_matches_finite_differences():
         assert abs(fd - float(dM[i, j])) < 1e-6 + 1e-4 * abs(fd)
 
 
-@pytest.mark.skipif(not os.path.exists(REFERENCE_FILE), reason="reference tree not present (GPU box)")
 def test_oracle_matches_live_reference_autograd():
-    ref = load_reference_module()
+    """Loss and autograd dL/dM of the reference Mapper's first epoch (random_state=5), from its own initial draw."""
+    g = np.load(os.path.join(GOLDEN_DIR, "live_reference_autograd.npz"))
     inp = synthetic_inputs(500, 130, 70, seed=9)
-    r = ref.Mapper(S=inp["S"], G=inp["G"], d=inp["d"], lambda_d=1.0, lambda_g2=0.2, lambda_r=1e-4,
-                   random_state=5)
-    M0 = r.M.detach().numpy().copy()
-    loss = r._loss_fn(verbose=False)[0]
-    loss.backward()
-    o = OracleMapper(inp["S"], inp["G"], d=inp["d"], lambda_d=1.0, lambda_g2=0.2, lambda_r=1e-4, M0=M0)
+    o = OracleMapper(inp["S"], inp["G"], d=inp["d"], lambda_d=1.0, lambda_g2=0.2, lambda_r=1e-4, random_state=5)
+    assert sha256_f32(o.M.numpy()) == str(g["M0_sha256"])        # the reference's draw, bit for bit
     terms, dM = o.loss_and_grad()
-    assert abs(terms["total_loss"] - float(loss)) < 2e-6
-    assert rel_fro(dM.numpy(), r.M.grad.numpy()) < 2e-5
+    assert abs(terms["total_loss"] - float(g["total_loss"])) < 2e-6
+    assert rel_fro(dM.numpy()[g["rows"]], g["grad_rows"]) < 2e-5
 
 
-@pytest.mark.skipif(not os.path.exists(REFERENCE_FILE), reason="reference tree not present (GPU box)")
 def test_unseeded_when_random_state_zero():
     """mapping_optimizer.py:148 -- random_state=0 is falsy -> no seeding (quirk preserved)."""
     inp = synthetic_inputs(8, 6, 5, seed=0)
@@ -97,17 +91,14 @@ def test_unseeded_when_random_state_zero():
     assert np.array_equal(a, b) and not np.array_equal(b, c)
 
 
-@pytest.mark.skipif(not os.path.exists(REFERENCE_FILE), reason="live reference not available")
 def test_second_train_call_restarts_adam_like_the_reference():
-    """mapping_optimizer.py:373: the optimizer is built inside train(), so a second call starts from zero moments."""
-    ref_mod = load_reference_module()
+    """mapping_optimizer.py:373: the optimizer is built inside train(), so a second call starts from zero moments.
+    Golden: the reference Mapper's second train(3) call after train(4)."""
+    g = np.load(os.path.join(GOLDEN_DIR, "live_reference_second_train.npz"))
     inp = synthetic_inputs(60, 25, 12, seed=4)
     kw = dict(S=inp["S"], G=inp["G"], d=inp["d"], lambda_d=1.0, random_state=7)
-    r = ref_mod.Mapper(device="cpu", **kw)
-    r.train(4, print_each=None)
-    r_out, r_hist = r.train(3, print_each=None)
     o = OracleMapper(**kw)
     o.train(4, print_each=None)
     o_out, o_hist = o.train(3, print_each=None)
-    assert rel_fro(o_out, r_out) < 1e-5
-    assert max_rel([float(x) for x in o_hist["total_loss"]], [float(x) for x in r_hist["total_loss"]]) < 1e-5
+    assert rel_fro(o_out, g["output"]) < 1e-5
+    assert max_rel([float(x) for x in o_hist["total_loss"]], g["total_loss"]) < 1e-5

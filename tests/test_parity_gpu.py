@@ -9,8 +9,8 @@ import numpy as np
 import pytest
 
 from oracle.tangram_oracle import OracleMapper, grid_graph, spatial_weights_from_graph, synthetic_inputs
-from tests.helpers import (assert_same_print, traj_err, GOLDEN_CASES, REFERENCE_FILE, load_golden, load_reference_module,
-                           max_rel, rel_fro)
+from tests.helpers import (assert_same_print, traj_err, GOLDEN_CASES, GOLDEN_DIR, load_golden, max_rel, rel_fro,
+                           sha256_f32)
 
 pytestmark = pytest.mark.gpu
 
@@ -168,26 +168,21 @@ def test_second_train_call_is_a_fresh_optimizer_like_the_reference():
     assert np.array_equal(a, b)
 
 
-@pytest.mark.skipif(not os.path.exists(REFERENCE_FILE), reason="reference file not available (oracle/build_ref.py)")
 def test_live_reference_on_the_same_gpu():
-    """The UNMODIFIED reference Mapper with device='cuda' (fp32 cuBLAS SGEMM, autograd, torch.optim.Adam) against the CUDA
-    path from the reference's own initial draw: loss trajectory and final mapping within north_star's 1e-4."""
-    import torch
-    ref = load_reference_module()
+    """The UNMODIFIED reference Mapper (fp32, autograd, torch.optim.Adam; golden from its CPU run,
+    tests/golden/make_live_reference_golden.py) against the CUDA path from the reference's own initial draw: loss
+    trajectory and final mapping (a fixed sample of 32 rows) within north_star's 1e-4."""
+    g = np.load(os.path.join(GOLDEN_DIR, "live_reference_30_epochs.npz"))
     inp = synthetic_inputs(3000, 700, 300, seed=31)
     kw = dict(S=inp["S"], G=inp["G"], d=inp["d"], lambda_d=1.0)
-    r = ref.Mapper(device="cuda:0", random_state=42, **kw)
-    M0 = r.M.detach().cpu().numpy().copy()
-    rout, rhist = r.train(num_epochs=30, learning_rate=0.1, print_each=None)
-    torch.cuda.synchronize()
+    # the default draw of the drop-in class is the reference's draw, bit for bit
+    M0 = _mapper(random_state=42, **kw).state()[0]
+    assert sha256_f32(M0) == str(g["M0_sha256"])
     m = _mapper(M0=M0, **kw)
     out, hist = m.train(30, print_each=None)
-    assert max_rel([float(x) for x in hist["total_loss"]], [float(x) for x in rhist["total_loss"]]) < 1e-4
-    assert max_rel(hist["main_loss"], rhist["main_loss"]) < 1e-4
-    assert rel_fro(out, rout) < 1e-4
-    # and the default draw of the drop-in class is the reference's draw, bit for bit
-    m2 = _mapper(random_state=42, **kw)
-    assert np.array_equal(m2.state()[0], M0)
+    assert max_rel([float(x) for x in hist["total_loss"]], g["total_loss"]) < 1e-4
+    assert max_rel(hist["main_loss"], g["main_loss"]) < 1e-4
+    assert rel_fro(out[g["rows"]], g["out_rows"]) < 1e-4
 
 
 def test_full_size_properties_config2():
